@@ -10,6 +10,7 @@ a small planted corpus: `merge_verified`).  Extra keys (N=1): BASELINE configs 3
 the 10M-doc strong-scaling legs.  Prints ONE JSON line (rank 0).
 
   python bench.py --gpus 1 --steps 10 --warmup 3
+  python bench.py --gpus 1 --steps 10 --warmup 3 --dump-outputs DIR   # + the last timed step's outputs as DIR/*.npy
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
   python bench.py --impl reference ...      # the reference's CPU path (HF GPTNeoModel fp32 + pooling + cos_sim/topk)
 """
@@ -300,6 +301,15 @@ def time_search(fn, steps, warm=3):
     return e0.elapsed_time(e1) / steps
 
 
+def dump_outputs(out_dir, arrays):
+    """`--dump-outputs DIR`: one DIR/<name>.npy per array (float32 / float64), so that two builds can be compared output
+    for output on the same seeded inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def other_config_legs(dev, pk, lib, steps):
     """BASELINE.json configs[2..4] at full size on ONE GPU (VERDICT r01 item 7): the encoder of each model at its batch x
     seq_len (random-init bf16 weights drawn on the GPU, inputs resident) and the exact top-1001 search over the shard
@@ -555,8 +565,8 @@ def run_b200(args, rank, world, local_rank):
     barrier()
 
     # ---- device-timed loop (inputs resident in HBM) -------------------------------------------------------------
-    # The timed region is K steps repeated R times back to back (R chosen so that the region lasts >= ~1.2 s: 30 steps of
-    # 7 ms alone would be a 0.2 s measurement); every number below is divided by K*R.  Two passes over the SAME steps:
+    # The timed region is the K = --steps steps back to back; every number below is divided by K (at ~7 ms a step, 30
+    # steps are a 0.2 s region: pass a larger --steps for a longer one).  Two passes over the SAME steps:
     # pass 1 is the timed region of `value` (three CUDA events per step); pass 2 repeats K steps with the library's
     # per-launch CUDA events switched on (two event records around each of the ~140 launches of a step cost ~7 % of the
     # step, so they stay out of pass 1) and feeds `roofline` / `kernel_ms_per_step`.
@@ -573,33 +583,30 @@ def run_b200(args, rank, world, local_rank):
         for k in range(n_steps):
             r = resident[k % len(resident)]
             ev[k][0].record()
-            enc.encode_packed(r[0], r[1], r[2], B, B * S, S)
+            emb = enc.encode_packed(r[0], r[1], r[2], B, B * S, S)
             ev[k][1].record()
-            search_step(queries)
+            s, i = search_step(queries)
             ev[k][2].record()
         barrier()
         t_w = time.perf_counter() - t_w0
         e_ms = sum(ev[k][0].elapsed_time(ev[k][1]) for k in range(n_steps))
         s_ms = sum(ev[k][1].elapsed_time(ev[k][2]) for k in range(n_steps))
-        return e_ms, s_ms, ev[0][0].elapsed_time(ev[-1][2]), t_w
+        return e_ms, s_ms, ev[0][0].elapsed_time(ev[-1][2]), t_w, (emb, s, i)
 
     K = args.steps
-    _, _, probe_ms, _ = timed_pass(min(K, 5))
-    step_est = maxr(probe_ms / min(K, 5))
-    R = max(1, int(np.ceil(1200.0 / max(1e-3, step_est * K))))
-    if world > 1:
-        rt = torch.tensor([R], device=dev)
-        dist.all_reduce(rt, op=dist.ReduceOp.MAX)
-        R = int(rt.item())
-    KR = K * R
     lib.sgpt_profile_read(None, None, tot_n0)
     lib.sgpt_profile_gemm_clock(ctypes.byref(gclk_c), ctypes.byref(gclk_ns))  # reset
-    enc_ms, sea_ms, tot_ms, t_wall = timed_pass(KR)
+    enc_ms, sea_ms, tot_ms, t_wall, (emb, s, i) = timed_pass(K)
     lib.sgpt_profile_read(None, None, tot_n1)
     lib.sgpt_profile_gemm_clock(ctypes.byref(gclk_c), ctypes.byref(gclk_ns))
     launches = sum(int(tot_n1[c] - tot_n0[c]) for c in range(8))
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path receives from its last step: the pooled embeddings and the search result
+        dump_outputs(args.dump_outputs, {"embeddings": emb.cpu().numpy(), "search_scores": s.cpu().numpy(),
+                                         "search_ids": i.cpu().double().numpy()})
+    del emb, s, i
     lib.sgpt_profile_enable(1)
-    _, _, prof_tot_ms, _ = timed_pass(K)
+    _, _, prof_tot_ms, _, _ = timed_pass(K)
     lib.sgpt_profile_enable(0)
     lib.sgpt_profile_read(prof_ms, prof_n, tot_n1)
 
@@ -657,8 +664,8 @@ def run_b200(args, rank, world, local_rank):
 
     # W untimed warm-up steps of exactly this loop first (host->device query copy, copies into the pinned result buffers)
     e2e_pass(True, max(args.warmup, 3))
-    e2e_s, h2d, d2h = e2e_pass(True, KR)
-    e2e_enc_s, _, _ = e2e_pass(False, KR)  # encode-only variant (extra key)
+    e2e_s, h2d, d2h = e2e_pass(True, K)
+    e2e_enc_s, _, _ = e2e_pass(False, K)  # encode-only variant (extra key)
 
     # the same search issued back to back (no encode in between): inside a step it starts in the clock / power state the
     # encoder leaves behind (SM and L2 clocks ~1.6 of 1.96 GHz under the power cap), which slows an HBM-streaming kernel
@@ -728,8 +735,8 @@ def run_b200(args, rank, world, local_rank):
         return
     pk = peaks()
     lin_flops, att_flops = encoder_flops_per_seq(S)
-    emb_per_s = world * B * KR / (enc_ms / 1e3)
-    qps = NQ * KR / (sea_ms / 1e3)
+    emb_per_s = world * B * K / (enc_ms / 1e3)
+    qps = NQ * K / (sea_ms / 1e3)
     gemm_ms, gemm_n = prof_ms[2], int(prof_n[2])
     gemm_tflops = (lin_flops * B * K) / (gemm_ms / 1e3) / 1e12 if gemm_ms > 0 else None
     att_ms = prof_ms[3]
@@ -740,7 +747,7 @@ def run_b200(args, rank, world, local_rank):
     # sampled tiles are scanned again by the filtered pass: <= 1/8, 3.7 % at this shape) — that re-read is overhead, not
     # credit: bytes per search / summed device time of both launches
     sim_gbs = sim_bytes * K / (sim_ms / 1e3) / 1e9 if sim_ms > 0 else None
-    whole_search_gbs = sim_bytes * KR / (sea_ms / 1e3) / 1e9
+    whole_search_gbs = sim_bytes * K / (sea_ms / 1e3) / 1e9
     traffic, traffic_src = measured_traffic()
     gemm_traffic = traffic.get("linear_gemm", {}).get("dram_bytes_per_launch")
     sim_traffic = traffic.get("similarity_gemm", {}).get("dram_bytes_per_launch")
@@ -754,11 +761,11 @@ def run_b200(args, rank, world, local_rank):
     gemm_launches_per_step = max(1, gemm_n // max(1, K))
     line = {
         "metric": METRIC, "value": emb_per_s, "unit": "embeddings/s", "n_gpus": world, "steps": K, "warmup": args.warmup,
-        "ms_per_step": tot_ms / KR, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "bf16",
+        "ms_per_step": tot_ms / K, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "bf16",
         "data": "synthetic", "config": workload_config(world),
-        "timed_region": {"repeats_of_the_K_steps": R, "steps_timed": KR, "device_seconds": tot_ms / 1e3,
+        "timed_region": {"steps_timed": K, "device_seconds": tot_ms / 1e3,
                          "note": "every per-step figure is the region's total divided by steps_timed"},
-        "encode_ms_per_step": enc_ms / KR, "search_ms_per_step": sea_ms / KR,
+        "encode_ms_per_step": enc_ms / K, "search_ms_per_step": sea_ms / K,
         "search": {"value": qps, "unit": "queries/s", "corpus_docs": NDOCS * world, "top_k": TOPK,
                    "pairs_per_s": qps * NDOCS * world, "exchange": transport,
                    "whole_search_frac_of_hbm": whole_search_gbs / pk["hbm"],
@@ -767,7 +774,7 @@ def run_b200(args, rank, world, local_rank):
                                     "note": "50 searches in a row, nothing else on the GPU; the step figure above is "
                                             "measured right after the encoder (power-capped clocks)"},
                    "large_query_batch": large},
-        "encoder_model_tflops": (lin_flops + att_flops) * B * world * KR / (enc_ms / 1e3) / 1e12,
+        "encoder_model_tflops": (lin_flops + att_flops) * B * world * K / (enc_ms / 1e3) / 1e12,
         "roofline": {"kernel": "gemm_bf16_tn_kernel (tcgen05 linear layers)", "bound": "tensor", "achieved": gemm_tflops,
                      "peak": pk["tf_sustained"], "unit": "TFLOP/s",
                      "frac": (gemm_tflops / pk["tf_sustained"]) if gemm_tflops else None, "traffic": gemm_traffic,
@@ -793,9 +800,9 @@ def run_b200(args, rank, world, local_rank):
         "profiled_pass_ms_per_step": prof_tot_ms / K,
         "gemm_sm_clock_mhz": (1e3 * gclk_c.value / gclk_ns.value) if gclk_ns.value > 0 else None,
         "gpu_launches": launches,
-        "e2e": {"value": world * B * KR / e2e_s, "unit": "embeddings/s", "h2d_bytes_per_step": h2d // KR,
-                "d2h_bytes_per_step": d2h // KR, "full_step_ms": 1000 * e2e_s / KR,
-                "encode_only_embeddings_per_s": world * B * KR / e2e_enc_s,
+        "e2e": {"value": world * B * K / e2e_s, "unit": "embeddings/s", "h2d_bytes_per_step": h2d // K,
+                "d2h_bytes_per_step": d2h // K, "full_step_ms": 1000 * e2e_s / K,
+                "encode_only_embeddings_per_s": world * B * K / e2e_enc_s,
                 "search_queries_per_s": None,
                 "note": "FULL step through the public API: Encoder.encode_tokens(host ids) -> embeddings copied into pinned "
                         "host memory, host->device queries, exact top-1001 search (+ cross-GPU exchange/merge at N>1), "
@@ -808,7 +815,7 @@ def run_b200(args, rank, world, local_rank):
         line["search_phases_ms"] = phases
     if big is not None:
         line["search_10m_strong_scaling"] = big
-    e2e_search_ms = 1000 * e2e_s / KR - 1000 * e2e_enc_s / KR
+    e2e_search_ms = 1000 * e2e_s / K - 1000 * e2e_enc_s / K
     line["e2e"]["search_queries_per_s"] = NQ / (e2e_search_ms / 1e3) if e2e_search_ms > 0 else None
     if cublas_cal is not None:
         line["roofline"]["cublas_same_shapes"] = cublas_cal
@@ -838,6 +845,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them returned to DIR/<name>.npy: embeddings "
+                         "(float32 [256, 768], rank 0's batch), search_scores (float32 [128, 1001]) and search_ids "
+                         "(float64 [128, 1001]); the inputs are seeded, so two builds can be compared output for output")
     ap.add_argument("--no-corpus-10m", dest="corpus_10m", action="store_false",
                     help="skip the extra legs that time the exact search over one 10M-doc corpus (D = 768 and 4096) split "
                          "across the ranks (strong scaling; reported as search_10m_strong_scaling)")
@@ -849,6 +860,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
         run_reference(args, rank)
         return
     if world > 1:

@@ -91,6 +91,12 @@ def write_modules_json(path, entries):
 
 def save_transformer(model, path, max_seq_length):
     model.save_pretrained(path)  # Transformer.save: auto_model.save_pretrained + tokenizer + sentence_bert_config.json
+    # the 2-D weights are bf16-exact (tiny_hf): stored as bf16 they keep every value in half the bytes (file < 1 MB)
+    from safetensors.torch import load_file, save_file
+
+    st = os.path.join(path, "model.safetensors")
+    save_file({k: v.to(torch.bfloat16) if v.dim() == 2 else v for k, v in load_file(st).items()}, st,
+              metadata={"format": "pt"})
     with open(os.path.join(path, "sentence_bert_config.json"), "w") as f:
         json.dump({"max_seq_length": max_seq_length, "do_lower_case": False}, f, indent=2)
 

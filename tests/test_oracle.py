@@ -218,7 +218,8 @@ def test_lm_score_oracle_matches_executed_reference_functions(golden_dir):
     from sgpt_b200.st_loader import load_torch_weights
 
     z = np.load(os.path.join(golden_dir, "ce_tiny.npz"))
-    w = load_torch_weights(os.path.join(golden_dir, "st_tiny"))
+    # the fixture stores its bf16-exact 2-D weights as bf16; the oracle computes in fp32
+    w = {k: v.float() for k, v in load_torch_weights(os.path.join(golden_dir, "st_tiny")).items()}
     spec = gpt_neo.NeoSpec(n_layer=2, d_model=128, n_head=2, d_ff=256, vocab=300, max_pos=64, window=8)
     reqs = _ce_requests(z)
     assert any(len(c) + len(q) > int(z["max_length"]) + 1 for _, c, q in reqs)  # truncation is exercised

@@ -1,21 +1,28 @@
-"""SURVEY.md §8f row 1 / VERDICT r01 item 9: the reference's own ``main`` (biencoder/beir/beir_dense_retriever.py:352-498)
-runs UNMODIFIED against the stand-in ``beir`` package and ``custommodels`` of sgpt_b200/compat.  This container has the
-reference but no GPU, so the two classes that launch CUDA kernels are replaced by CPU stand-ins that keep their
-interfaces (a toy embedder with CustomEmbedder's constructor keywords; the oracle's restatement of the search loop behind
-DenseRetrievalExactSearch's ``search``); everything else — argument parsing, GenericDataLoader, empty-text filtering,
-EvaluateRetrieval.retrieve/evaluate, the result and metric files — is the reference's code driving the stand-in
-package.  (On the GPU box the reference is absent; the same flow with the real classes is covered by
-tests/test_gpu_heads.py and `python -m sgpt_b200.compat.run_reference`.)"""
+"""SURVEY.md §8f row 1 / VERDICT r01 item 9: the retrieval run of the original project's
+biencoder/beir/beir_dense_retriever.py (its ``main``, BDR:352-498) against ``sgpt_b200.retrieve.main`` on one toy BEIR
+dataset.  tests/golden/reference_main_toyset.json holds the two files the original ``main`` wrote when it ran unmodified
+on the stand-in ``beir`` package and ``custommodels`` of sgpt_b200/compat (tests/golden/make_reference_main.py), and
+every name the script imports from those two packages.  The test checks that those imports resolve in the stand-in
+packages through ``load_reference_script``, and that ``sgpt_b200.retrieve.main`` writes the same result file (same
+documents and scores per query) and the same metrics file.  In both runs the two classes that launch CUDA kernels are
+replaced by CPU stand-ins that keep their interfaces (a toy embedder with CustomEmbedder's constructor keywords; the
+oracle's restatement of the search loop behind DenseRetrievalExactSearch's ``search``); everything else — argument
+parsing, GenericDataLoader, empty-text filtering, EvaluateRetrieval.retrieve/evaluate, the result and metric files — is
+the code under comparison.  (The same flow with the real classes is covered by tests/test_gpu_heads.py.)"""
 import json
 import os
 import sys
 import zlib
 
 import numpy as np
-import pytest
 import torch
 
-REF = "/root/reference/biencoder/beir/beir_dense_retriever.py"
+from tests.conftest import GOLDEN
+
+GOLDEN_FILE = os.path.join(GOLDEN, "reference_main_toyset.json")
+# command line of both runs; --datapath (and --outdir for sgpt_b200.retrieve) are added per run
+ARGV = ["--dataset", "toyset", "--modelname", "toy/model", "--method", "weightedmean", "--device", "cpu",
+        "--batchsize", "16", "--specb"]
 
 
 class _ToyEmbedder:
@@ -65,54 +72,83 @@ class _CpuDRES:
         return self.results
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="the reference tree is only present in the build container")
-def test_reference_main_runs_unmodified_on_the_stand_in_packages(tmp_path, monkeypatch):
-    from sgpt_b200 import compat
-    from sgpt_b200.compat.run_reference import load_reference_script
-
-    # toy BEIR directory: the relevant document of every query repeats the query's words
+def write_toyset(datasets_dir):
+    """Toy BEIR directory ``<datasets_dir>/toyset``: the relevant document of every query repeats the query's words, and
+    one document has an empty text.  Returns the queries."""
     rs = np.random.RandomState(0)
     words = [f"w{i}" for i in range(200)]
-    root = tmp_path / "datasets" / "toyset"
-    os.makedirs(root / "qrels")
+    root = os.path.join(datasets_dir, "toyset")
+    os.makedirs(os.path.join(root, "qrels"))
     corpus = {f"d{i}": {"title": " ".join(rs.choice(words, 2)), "text": " ".join(rs.choice(words, rs.randint(3, 30)))}
               for i in range(60)}
     corpus["d_empty"] = {"title": "t", "text": ""}  # removed by the script (BDR:382-388)
     queries = {f"q{i}": corpus[f"d{i}"]["text"] for i in range(8)}
-    with open(root / "corpus.jsonl", "w") as f:
+    with open(os.path.join(root, "corpus.jsonl"), "w") as f:
         for k, v in corpus.items():
             f.write(json.dumps({"_id": k, **v}) + "\n")
-    with open(root / "queries.jsonl", "w") as f:
+    with open(os.path.join(root, "queries.jsonl"), "w") as f:
         for k, v in queries.items():
             f.write(json.dumps({"_id": k, "text": v}) + "\n")
-    with open(root / "qrels" / "test.tsv", "w") as f:
+    with open(os.path.join(root, "qrels", "test.tsv"), "w") as f:
         f.write("query-id\tcorpus-id\tscore\n")
         for i in range(8):
             f.write(f"q{i}\td{i}\t1\n")
+    return queries
 
-    monkeypatch.chdir(tmp_path)  # the script writes its result files into the working directory
+
+def _assert_close(got, want, path="scores"):
+    """Same nested keys; numbers within 1e-6 (metrics are rounded to 5 decimals, scores are fp32 cosines)."""
+    if isinstance(want, dict):
+        assert isinstance(got, dict) and set(got) == set(want), f"{path}: keys {sorted(got)} != {sorted(want)}"
+        for k in want:
+            _assert_close(got[k], want[k], f"{path}/{k}")
+    else:
+        assert abs(got - want) <= 1e-6, f"{path}: {got} != {want}"
+
+
+def test_retrieve_main_matches_reference_main_on_the_stand_in_packages(tmp_path, monkeypatch):
+    import sgpt_b200
+    from sgpt_b200 import compat, retrieve
+    from sgpt_b200.compat.run_reference import load_reference_script
+
+    with open(GOLDEN_FILE) as f:
+        want = json.load(f)
+    queries = write_toyset(str(tmp_path / "datasets"))
+
+    # the original script's imports from `beir` / `custommodels`, loaded the way run_reference loads the script
+    script = tmp_path / "imports_of_the_reference_script.py"
+    script.write_text("".join(f"from {mod} import {name}\n" for mod, names in want["imports"] for name in names)
+                      + "\n\nclass CustomEmbedder:\n    pass\n")
     monkeypatch.setattr(sys, "path", list(sys.path))
-    mod = load_reference_script(REF, embedder_cls=_ToyEmbedder, module_name="ref_bdr_under_test")
+    mod = load_reference_script(str(script), embedder_cls=_ToyEmbedder, module_name="ref_bdr_imports_under_test")
+    assert mod.CustomEmbedder is _ToyEmbedder
     import beir
     import custommodels
 
     assert os.path.dirname(os.path.dirname(beir.__file__)) == compat.COMPAT_DIR  # the stand-in, not an installed beir
-    monkeypatch.setattr(mod, "DenseRetrievalExactSearch", _CpuDRES)  # (bound at import: `from custommodels import ...`)
     assert custommodels.DenseRetrievalExactSearch.__module__ == "sgpt_b200.exact_search"
-    monkeypatch.setattr(sys, "argv", ["beir_dense_retriever.py", "--dataset", "toyset", "--datapath", str(tmp_path / "datasets"),
-                                      "--modelname", "toy/model", "--method", "weightedmean", "--device", "cpu",
-                                      "--batchsize", "16", "--specb"])
-    args = mod.parse_args()
-    mod.main(args)
 
-    results = json.load(open(tmp_path / "results_toy_model_weightedmean_toyset.json"))
+    # the project's retrieval run, with the same two CPU stand-ins the original run had
+    monkeypatch.setattr(sgpt_b200, "CustomEmbedder", _ToyEmbedder)
+    monkeypatch.setattr(sgpt_b200, "DenseRetrievalExactSearch", _CpuDRES)
+    out = tmp_path / "out"
+    out.mkdir()
+    args = retrieve.parse_args(ARGV + ["--datapath", str(tmp_path / "datasets"), "--outdir", str(out)])
+    retrieve.main(args)
+
+    assert sorted(os.listdir(out)) == sorted([want["result_file"], "beir_embeddings_ndcgs.json"])
+    with open(out / want["result_file"]) as f:
+        results = json.load(f)
+    _assert_close(results, want["results"], "results")
+    with open(out / "beir_embeddings_ndcgs.json") as f:
+        nd = json.load(f)
+    _assert_close(nd, want["scores"])
     assert set(results) == set(queries)
     for i in range(8):
         assert max(results[f"q{i}"], key=results[f"q{i}"].get) == f"d{i}"  # the planted document ranks first
         assert "d_empty" not in results[f"q{i}"]
-    nd = json.load(open(tmp_path / "beir_embeddings_ndcgs.json"))
     assert nd["ndcgs"]["toy_model"]["toyset"]["NDCG@1"] == 1.0
     assert nd["recalls"]["toy_model"]["toyset"]["Recall@10"] == 1.0
     assert set(nd) >= {"ndcgs", "maps", "recalls", "precisions"}
     # a second run finds the result file and skips (BDR:433-436)
-    mod.main(args)
+    assert retrieve.main(args) == {}
