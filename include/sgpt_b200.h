@@ -250,6 +250,20 @@ int sgpt_row_inv_norms(const void* x, float* inv_norm, int64_t n, int D, sgpt_st
 /* fp32 -> bf16 row conversion (round-to-nearest-even) used to store embeddings in a shard. */
 int sgpt_f32_to_bf16(const float* x, void* y, int64_t count, sgpt_stream_t stream);
 
+/* Element types of a corpus shard (and of the queries searched against it): the `elem` argument of the _ex entry
+ * points below.  SGPT_ELEM_I8 = int8 rows quantized per row by sgpt_quantize_rows_i8 (D a multiple of 16, D <= 65536). */
+#define SGPT_ELEM_BF16 0
+#define SGPT_ELEM_I8 1
+
+/* Symmetric per-row int8 quantization, for corpus rows and query rows alike.  x fp32[n,D] (x_is_bf16 = 0) or bf16[n,D]
+ * (x_is_bf16 = 1, widened exactly); per row: s = max_j |x_j| / 127 (IEEE fp32), c_j = clamp(rint(x_j / s), -127, 127)
+ * (round-half-even; s = 0 gives c = 0), inv = 1 / max(sqrt((float)sum_j c_j^2), 1e-12).  out int8[n,D], scale fp32[n]
+ * = s, inv_norm fp32[n] = inv.  An int8 search then scores cos_sim = ((float)acc * inv_q) * inv_d and
+ * dot = ((float)acc * s_q) * s_d with acc = sum_j cq_j cd_j exact in int32: cos_sim / dot_score of the dequantized rows
+ * s * c.  Rows must be finite (not checked here: the Python layer rejects non-finite rows).  D % 16 == 0, D <= 65536. */
+int sgpt_quantize_rows_i8(const void* x, int x_is_bf16, int64_t n, int D, int8_t* out, float* scale, float* inv_norm,
+                          sgpt_stream_t stream);
+
 /* S1. scores[q,j] = fixnan( <Q[q,:], C[j,:]> * q_scale[q] * c_scale[j] )      ST/util.py:24-63, XS:96-99
  *     Q bf16[nq,D], C bf16[n,D], q_scale fp32[nq]|NULL, c_scale fp32[n]|NULL (NULL = 1: dot_score),
  *     scores fp32[nq, lds]; NaN -> -1 as XS:99.  tcgen05 GEMM, corpus streamed once from HBM. */
@@ -285,6 +299,16 @@ int sgpt_search(const void* Q, const void* C, const float* q_scale, const float*
 int sgpt_search_packed(const void* Q, const void* C, const float* q_scale, const float* c_scale, int nq, int64_t n,
                        int D, int k, int64_t id_base, uint64_t* out_packed, void* ws, int64_t ws_bytes,
                        sgpt_stream_t stream);
+/* sgpt_search / sgpt_search_packed for either element type (SGPT_ELEM_BF16: identical to the calls above;
+ * SGPT_ELEM_I8: Q int8[nq,D] and C int8[n,D] from sgpt_quantize_rows_i8, q_scale / c_scale = the inverse norms for
+ * cos_sim or the scales for dot).  Same workspace size for both types.  SGPT_ERR_INVALID before any CUDA call for an
+ * unknown elem, an int8 D that is not a multiple of 16 or exceeds 65536, or a null output. */
+int sgpt_search_ex(const void* Q, const void* C, const float* q_scale, const float* c_scale, int nq, int64_t n, int D,
+                   int k, int64_t id_base, float* out_scores, int64_t* out_ids, void* ws, int64_t ws_bytes, int elem,
+                   sgpt_stream_t stream);
+int sgpt_search_packed_ex(const void* Q, const void* C, const float* q_scale, const float* c_scale, int nq, int64_t n,
+                          int D, int k, int64_t id_base, uint64_t* out_packed, void* ws, int64_t ws_bytes, int elem,
+                          sgpt_stream_t stream);
 /* S3 on packed lists: in_packed uint64[G,nq,k] (the all-gathered sgpt_search_packed outputs; chunk = shard in
  *     XS:121-132) -> out_scores fp32[nq,k], out_ids int64[nq,k]; ids < 0 and ids == exclude_ids[q] (XS:118) dropped.
  *     Every input list must be in the order sgpt_search_packed writes (score descending, id ascending on ties, empty
@@ -313,6 +337,11 @@ void sgpt_gather_destroy(sgpt_gather_t g);
 int sgpt_search_gather(sgpt_gather_t g, const void* Q, const void* C, const float* q_scale, const float* c_scale,
                        int nq, int64_t n, int D, int k, int64_t id_base, const int64_t* exclude_ids, float* out_scores,
                        int64_t* out_ids, void* ws, int64_t ws_bytes, sgpt_stream_t stream);
+/* sgpt_search_gather for either element type (elem and its checks as sgpt_search_ex). */
+int sgpt_search_gather_ex(sgpt_gather_t g, const void* Q, const void* C, const float* q_scale, const float* c_scale,
+                          int nq, int64_t n, int D, int k, int64_t id_base, const int64_t* exclude_ids,
+                          float* out_scores, int64_t* out_ids, void* ws, int64_t ws_bytes, int elem,
+                          sgpt_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
  * Residual stream in bf16 (SGPT_RESID_BF16=1 when the model handle is created; default fp32).  HF keeps hidden_states in

@@ -18,6 +18,7 @@ EPI_BF16, EPI_GELU_BF16, EPI_RESID_F32, EPI_RESID_BF16 = 0, 1, 2, 3
 POOL_MEAN, POOL_WEIGHTEDMEAN, POOL_LASTTOKEN, POOL_MEANMEAN, POOL_LASTTOKENMEAN = 0, 1, 2, 3, 4
 ARCH_GPT_NEO, ARCH_GPTJ, ARCH_BLOOM = 0, 1, 2
 ACT_IDENTITY, ACT_TANH, ACT_RELU, ACT_SIGMOID = 0, 1, 2, 3
+ELEM_BF16, ELEM_I8 = 0, 1  # element type of a corpus shard (SGPT_ELEM_*)
 
 i32, i64, f32, vp = C.c_int32, C.c_int64, C.c_float, C.c_void_p
 
@@ -93,6 +94,10 @@ _SIGNATURES = {
     "sgpt_gather_connect": (i32, [vp, vp]),
     "sgpt_gather_destroy": (None, [vp]),
     "sgpt_search_gather": (i32, [vp, vp, vp, vp, vp, i32, i64, i32, i32, i64, vp, vp, vp, vp, i64, vp]),
+    "sgpt_quantize_rows_i8": (i32, [vp, i32, i64, i32, vp, vp, vp, vp]),
+    "sgpt_search_ex": (i32, [vp, vp, vp, vp, i32, i64, i32, i32, i64, vp, vp, vp, i64, i32, vp]),
+    "sgpt_search_packed_ex": (i32, [vp, vp, vp, vp, i32, i64, i32, i32, i64, vp, vp, i64, i32, vp]),
+    "sgpt_search_gather_ex": (i32, [vp, vp, vp, vp, vp, i32, i64, i32, i32, i64, vp, vp, vp, vp, i64, i32, vp]),
 }
 
 ABI_VERSION = 3  # include/sgpt_b200.h SGPT_ABI_VERSION these signatures / struct layouts were written for

@@ -315,6 +315,28 @@ __device__ __forceinline__ void umma_bf16_ss_pair(uint32_t tmem_d, uint64_t desc
       : "r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// int8 operands (signed x signed), s32 accumulate: K = 32 per instruction, i.e. the same 32 bytes of a 128-byte swizzle
+// row as a K = 16 bf16 MMA, so the smem descriptors and their +2 advance are shared with the bf16 forms.
+__device__ __forceinline__ void umma_s8_ss(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                           uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}\n"
+      :
+      : "r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void umma_s8_ss_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                                uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t}\n"
+      :
+      : "r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // Arrive (once all previously issued pair MMAs completed) on the barrier at this smem offset in the CTAs of cta_mask.
 __device__ __forceinline__ void umma_commit_pair(uint64_t* bar, uint16_t cta_mask) {
   asm volatile(
@@ -364,6 +386,14 @@ __device__ __forceinline__ void tma_load_2d_pair_multicast(void* smem_dst, const
 __host__ __device__ constexpr uint32_t make_idesc_bf16(int m, int n, bool b_mn_major) {
   return (1u << 4) | (1u << 7) | (1u << 10) | (0u << 15) | ((b_mn_major ? 1u : 0u) << 16) |
          (static_cast<uint32_t>(n >> 3) << 17) | (static_cast<uint32_t>(m >> 4) << 24);
+}
+
+// Instruction descriptor for kind::i8 with signed 8-bit A/B, s32 D, both operands K-major.
+//   [4,6) D format (2 = s32)   [7,10) A format (1 = signed 8-bit)   [10,13) B format (1 = signed 8-bit)
+//   [13,15) negate A/B (must be 0 for kind::i8)   [17,23) N >> 3   [24,29) M >> 4
+__host__ __device__ constexpr uint32_t make_idesc_s8(int m, int n) {
+  return (2u << 4) | (1u << 7) | (1u << 10) | (static_cast<uint32_t>(n >> 3) << 17) |
+         (static_cast<uint32_t>(m >> 4) << 24);
 }
 
 // Shared-memory matrix descriptor, SWIZZLE_128B, for tiles written by TMA with a 128-byte inner box.

@@ -791,6 +791,74 @@ __global__ void __launch_bounds__(256) row_inv_norm_kernel(const uint4* __restri
   if (lane == 0) inv[row] = 1.0f / fmaxf(sqrtf(s), 1e-12f);
 }
 
+// Symmetric per-row int8 quantization of int8 corpus shards and their queries (include/sgpt_b200.h
+// sgpt_quantize_rows_i8 states the arithmetic; the CPU oracle in tests/int8_oracle.py reproduces it bit for bit, which is
+// why every step is an explicitly IEEE-rounded intrinsic).  One warp per row, 16 elements per lane step (4 x 16-byte fp32
+// loads or 2 x 16-byte bf16 loads, one 16-byte store).  The row is read twice — the maximum first, then the quantization —
+// and the second read is served by the L2 that the first one filled.  D % 16 == 0.
+template <bool kBF16>
+__device__ __forceinline__ void load_row16(const void* x, long long i16, float (&v)[16]) {
+  if constexpr (kBF16) {
+    const uint4* p = static_cast<const uint4*>(x) + i16 * 2;
+    const uint4 a = __ldg(p), b = __ldg(p + 1);
+    const uint32_t u[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      v[2 * j] = bf16_lo(u[j]);
+      v[2 * j + 1] = bf16_hi(u[j]);
+    }
+  } else {
+    const float4* p = static_cast<const float4*>(x) + i16 * 4;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const float4 f = __ldg(p + j);
+      v[4 * j] = f.x;
+      v[4 * j + 1] = f.y;
+      v[4 * j + 2] = f.z;
+      v[4 * j + 3] = f.w;
+    }
+  }
+}
+
+template <bool kBF16>
+__global__ void __launch_bounds__(256) quantize_rows_i8_kernel(const void* __restrict__ x, uint4* __restrict__ out,
+                                                               float* __restrict__ scale, float* __restrict__ inv,
+                                                               long long n, int d16) {
+  pdl_sync();  // programmatic dependent launch: see common.cuh
+  const long long row = blockIdx.x * 8ll + (threadIdx.x >> 5);
+  if (row >= n) return;
+  const int lane = threadIdx.x & 31;
+  float a = 0.f;
+  for (int c = lane; c < d16; c += 32) {
+    float v[16];
+    load_row16<kBF16>(x, row * d16 + c, v);
+#pragma unroll
+    for (int i = 0; i < 16; ++i) a = fmaxf(a, fabsf(v[i]));
+  }
+  a = warp_max(a);
+  const float s = __fdiv_rn(a, 127.0f);
+  int n2 = 0;
+  for (int c = lane; c < d16; c += 32) {
+    float v[16];
+    load_row16<kBF16>(x, row * d16 + c, v);
+    uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+    for (int i = 0; i < 16; ++i) {
+      // s == 0 only for an all-zero row (or one whose maximum underflows): every code is 0 then
+      const int q = s > 0.f ? static_cast<int>(fminf(fmaxf(rintf(__fdiv_rn(v[i], s)), -127.f), 127.f)) : 0;
+      n2 += q * q;
+      w[i >> 2] |= (static_cast<uint32_t>(q) & 0xffu) << (8 * (i & 3));
+    }
+    out[row * d16 + c] = make_uint4(w[0], w[1], w[2], w[3]);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) n2 += __shfl_xor_sync(0xffffffffu, n2, o);  // exact: n2 <= 127^2 x 65536 < 2^31
+  if (lane == 0) {
+    scale[row] = s;
+    inv[row] = __fdiv_rn(1.0f, fmaxf(__fsqrt_rn(__int2float_rn(n2)), 1e-12f));
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // Sentence-embedding head: y[b,o] = act(sum_k x[b,k] * w[o,k] + bias[o]) in fp32 (ST/models/Dense.py:40-43 applied to
 // the pooled embedding).  B x in x out is tiny (<= a few hundred MFLOP), so this is a plain smem-tiled SIMT kernel kept
@@ -1149,5 +1217,22 @@ extern "C" int sgpt_f32_to_bf16(const float* x, void* y, int64_t count, sgpt_str
   LaunchScope _ls(kCatMisc, stream);
   SGPT_CHECK_CUDA(launch_kernel(f32_to_bf16_kernel, dim3(grid_for(count / 4, 256)), dim3(256), 0, stream,
                                 reinterpret_cast<const float4*>(x), static_cast<uint2*>(y), count / 4));
+  return SGPT_OK;
+}
+
+extern "C" int sgpt_quantize_rows_i8(const void* x, int x_is_bf16, int64_t n, int D, int8_t* out, float* scale,
+                                     float* inv_norm, sgpt_stream_t stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  SGPT_REQUIRE(n >= 0 && D > 0 && D % 16 == 0 && D <= 65536,
+               "sgpt_quantize_rows_i8: D=%d must be a positive multiple of 16 and <= 65536 (n=%lld)", D, (long long)n);
+  SGPT_REQUIRE(n == 0 || (x != nullptr && out != nullptr && scale != nullptr && inv_norm != nullptr),
+               "sgpt_quantize_rows_i8: null argument");
+  if (n == 0) return SGPT_OK;
+  const long long blocks = (n + 7) / 8;
+  SGPT_REQUIRE(blocks < (1ll << 31), "sgpt_quantize_rows_i8: too many rows");
+  LaunchScope _ls(kCatMisc, stream);
+  auto kern = x_is_bf16 ? quantize_rows_i8_kernel<true> : quantize_rows_i8_kernel<false>;
+  SGPT_CHECK_CUDA(launch_kernel(kern, dim3(static_cast<unsigned>(blocks)), dim3(256), 0, stream, x,
+                                reinterpret_cast<uint4*>(out), scale, inv_norm, static_cast<long long>(n), D / 16));
   return SGPT_OK;
 }

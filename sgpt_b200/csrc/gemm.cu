@@ -12,21 +12,21 @@
 
 namespace sgpt {
 
-template <int BN, class Epi, int CL = 1>
+template <int BN, class Epi, int CL = 1, int kOperand = kOperandBF16>
 static int launch_gemm(const void* a, int64_t lda, const void* b, int64_t ldb, int M, int N, int K,
                        const typename Epi::Params& ep, cudaStream_t stream, int cat = kCatGemm,
                        TileMap tmap = TileMap()) {
   using Cfg = GemmCfg<BN, CL, EpiStaging<Epi>::value>;
+  constexpr int kBK = OperandTraits<kOperand>::kBK;  // one 128-byte row segment: 64 bf16 or 128 int8
+  auto make_map = kOperand == kOperandS8 ? make_tma_2d_u8 : make_tma_2d_bf16;
   CUtensorMap ta, tb;
-  int rc = make_tma_2d_bf16(&ta, a, static_cast<uint64_t>(M), static_cast<uint64_t>(K), static_cast<uint64_t>(lda),
-                            kGemmBM, kGemmBK);
+  int rc = make_map(&ta, a, static_cast<uint64_t>(M), static_cast<uint64_t>(K), static_cast<uint64_t>(lda), kGemmBM, kBK);
   if (rc != SGPT_OK) return rc;
   // in a CTA pair each CTA holds half of the B tile; with two pairs per cluster (CL = 4) it fetches a quarter and
   // receives the other quarter of its half by multicast from the CTA of its parity in the other pair
-  rc = make_tma_2d_bf16(&tb, b, static_cast<uint64_t>(N), static_cast<uint64_t>(K), static_cast<uint64_t>(ldb), BN / CL,
-                        kGemmBK);
+  rc = make_map(&tb, b, static_cast<uint64_t>(N), static_cast<uint64_t>(K), static_cast<uint64_t>(ldb), BN / CL, kBK);
   if (rc != SGPT_OK) return rc;
-  auto kern = gemm_bf16_tn_kernel<BN, Epi, CL>;
+  auto kern = gemm_bf16_tn_kernel<BN, Epi, CL, kOperand>;
   static PerDeviceOnce attr_once;
   if (attr_once.first()) {
     SGPT_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes));
@@ -187,17 +187,24 @@ FilterGeometry filter_geometry(long long tiles, int nq) {
 
 // nq <= 128: independent CTAs (M = 128).  128 < nq <= 256: CTA pairs running tcgen05.mma.cta_group::2 with M = 256 — each CTA
 // holds 128 of the queries and HALF of every corpus tile, so a scan moves half the corpus bytes per query through each SM
-// and the kernel turns from HBM-bound into tensor-bound (2 x the queries per pass over the shard).
+// and the kernel turns from HBM-bound into tensor-bound (2 x the queries per pass over the shard).  elem selects bf16 or
+// int8 operands (kind::f16 / kind::i8; the epilogue then converts the s32 accumulator).
 template <class P>
-static int launch_filter_gemm(const void* Q, const void* C, int nq, int n, int D, const P& p, cudaStream_t stream, TileMap tm) {
+static int launch_filter_gemm(const void* Q, const void* C, int nq, int n, int D, int elem, const P& p,
+                              cudaStream_t stream, TileMap tm) {
+  if (elem == SGPT_ELEM_I8) {
+    if (nq > kGemmBM)
+      return launch_gemm<kSimBN, EpiFilterRowsS8, 2, kOperandS8>(Q, D, C, D, nq, n, D, p, stream, kCatScores, tm);
+    return launch_gemm<kSimBN, EpiFilterRowsS8, 1, kOperandS8>(Q, D, C, D, nq, n, D, p, stream, kCatScores, tm);
+  }
   if (nq > kGemmBM) return launch_gemm<kSimBN, EpiFilterRows, 2>(Q, D, C, D, nq, n, D, p, stream, kCatScores, tm);
   return launch_gemm<kSimBN, EpiFilterRows, 1>(Q, D, C, D, nq, n, D, p, stream, kCatScores, tm);
 }
 
 int launch_filter_candidates(const void* Q, const void* C, const float* q_scale, const float* c_scale,
                              const float* tau, const float* tau_hi, uint2* cand, int* counts, int* counts_back,
-                             long long stride_q, int L, int group0, int nq, int n, int D, int tile_mode, int tile_stride,
-                             cudaStream_t stream) {
+                             long long stride_q, int L, int group0, int nq, int n, int D, int elem, int tile_mode,
+                             int tile_stride, cudaStream_t stream) {
   SGPT_REQUIRE(nq <= 2 * kGemmBM, "filter GEMM: at most %d queries per launch (got %d)", 2 * kGemmBM, nq);
   TileMap tm;
   tm.mode = tile_mode;
@@ -207,11 +214,12 @@ int launch_filter_candidates(const void* Q, const void* C, const float* q_scale,
                g.L);
   EpiFilterRows::Params p{q_scale, c_scale, tau, tau_hi, cand, counts, counts_back, stride_q, L, group0, nq, nullptr, 0, 0,
                           nq > kGemmBM ? 1 : 0};
-  return launch_filter_gemm(Q, C, nq, n, D, p, stream, tm);
+  return launch_filter_gemm(Q, C, nq, n, D, elem, p, stream, tm);
 }
 
 int launch_sample_maxima(const void* Q, const void* C, const float* q_scale, const float* c_scale, float* pool,
-                         long long stride_p, int Lp, int nq, int n, int D, int tile_stride, cudaStream_t stream) {
+                         long long stride_p, int Lp, int nq, int n, int D, int elem, int tile_stride,
+                         cudaStream_t stream) {
   SGPT_REQUIRE(nq <= 2 * kGemmBM, "sample GEMM: at most %d queries per launch (got %d)", 2 * kGemmBM, nq);
   TileMap tm;
   tm.mode = 1;
@@ -221,7 +229,22 @@ int launch_sample_maxima(const void* Q, const void* C, const float* q_scale, con
                "sample GEMM: maxima lists too small (Lp=%d < %d)", Lp, g.L / 4);
   EpiFilterRows::Params p{q_scale, c_scale, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0, 0, nq, pool, stride_p, Lp,
                           nq > kGemmBM ? 1 : 0};
-  return launch_filter_gemm(Q, C, nq, n, D, p, stream, tm);
+  return launch_filter_gemm(Q, C, nq, n, D, elem, p, stream, tm);
+}
+
+int launch_scores(const void* Q, const void* C, const float* q_scale, const float* c_scale, float* scores, int64_t lds,
+                  int nq, int64_t n, int D, int elem, cudaStream_t stream) {
+  SGPT_REQUIRE(nq >= 0 && n >= 0 && D > 0 && D % 8 == 0, "sgpt_scores: bad sizes nq=%d n=%lld D=%d", nq,
+               (long long)n, D);
+  SGPT_REQUIRE(n < (1ll << 31), "sgpt_scores: shard too large for one launch (n=%lld)", (long long)n);
+  SGPT_REQUIRE(lds >= n, "sgpt_scores: lds < n");
+  if (nq == 0 || n == 0) return SGPT_OK;
+  EpiScoresF32::Params p{scores, q_scale, c_scale, static_cast<long long>(lds)};
+  // lanes = queries (A operand), columns = corpus rows (B operand, streamed once from HBM)
+  if (elem == SGPT_ELEM_I8)
+    return launch_gemm<kSimBN, EpiScoresF32S8, 1, kOperandS8>(Q, D, C, D, nq, static_cast<int>(n), D, p, stream,
+                                                              kCatScores);
+  return launch_gemm<kSimBN, EpiScoresF32>(Q, D, C, D, nq, static_cast<int>(n), D, p, stream, kCatScores);
 }
 
 }  // namespace sgpt
@@ -431,13 +454,5 @@ extern "C" int sgpt_linear_resid_ln(const void* x, int64_t ldx, const void* w, i
 
 extern "C" int sgpt_scores(const void* Q, const void* C, const float* q_scale, const float* c_scale, float* scores,
                            int64_t lds, int nq, int64_t n, int D, sgpt_stream_t stream_) {
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  SGPT_REQUIRE(nq >= 0 && n >= 0 && D > 0 && D % 8 == 0, "sgpt_scores: bad sizes nq=%d n=%lld D=%d", nq,
-               (long long)n, D);
-  SGPT_REQUIRE(n < (1ll << 31), "sgpt_scores: shard too large for one launch (n=%lld)", (long long)n);
-  SGPT_REQUIRE(lds >= n, "sgpt_scores: lds < n");
-  if (nq == 0 || n == 0) return SGPT_OK;
-  EpiScoresF32::Params p{scores, q_scale, c_scale, static_cast<long long>(lds)};
-  // lanes = queries (A operand), columns = corpus rows (B operand, streamed once from HBM)
-  return launch_gemm<kSimBN, EpiScoresF32>(Q, D, C, D, nq, static_cast<int>(n), D, p, stream, kCatScores);
+  return launch_scores(Q, C, q_scale, c_scale, scores, lds, nq, n, D, SGPT_ELEM_BF16, static_cast<cudaStream_t>(stream_));
 }

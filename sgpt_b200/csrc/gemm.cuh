@@ -1,4 +1,5 @@
-// Persistent, warp-specialised tcgen05 GEMM for sm_100a:  C[M,N] = A[M,K] * B[N,K]^T  (bf16 in, fp32 accumulate).
+// Persistent, warp-specialised tcgen05 GEMM for sm_100a:  C[M,N] = A[M,K] * B[N,K]^T  (bf16 in, fp32 accumulate; the
+// similarity scans of int8 corpus shards: int8 in, s32 accumulate, see kOperandS8).
 //
 //   A : activations / queries, row-major [M,K]  -> K-major UMMA operand A (TMEM lane = row of A)
 //   B : nn.Linear weight [out,in] / corpus shard [n,D], row-major [N,K] -> K-major UMMA operand B
@@ -29,6 +30,25 @@ namespace sgpt {
 
 constexpr int kGemmBM = 128;
 constexpr int kGemmBK = 64;
+
+// Operand kind of the persistent GEMM.  A k-block is one 128-byte SWIZZLE_128B row either way: 64 bf16 (kind::f16,
+// K = 16 per MMA, fp32 accumulator) or 128 int8 (kind::i8, K = 32 per MMA, s32 accumulator); stage sizes, smem
+// descriptors and their advance are the same.  Epilogues of int8 launches convert the s32 accumulator with acc_to_f32.
+constexpr int kOperandBF16 = 0;
+constexpr int kOperandS8 = 1;
+template <int kOperand>
+struct OperandTraits {
+  static constexpr int kBK = kGemmBK;  // elements per k-block
+};
+template <>
+struct OperandTraits<kOperandS8> {
+  static constexpr int kBK = 2 * kGemmBK;
+};
+template <bool kS8>
+__device__ __forceinline__ float acc_to_f32(uint32_t v) {
+  if constexpr (kS8) return __int2float_rn(static_cast<int>(v));
+  else return __uint_as_float(v);
+}
 constexpr int kGemmThreads = 256;
 constexpr int kStageBytesPerWarp = 8192;  // per epilogue warp: 2 TMA boxes of 32 x 128 B, or one 32 x 64 fp32 slab
 
@@ -143,7 +163,8 @@ struct TileMap {
 //   the CTA of the same parity in the other pair: per k-block the four CTAs read 64 KB of A + 32 KB of B from L2 instead
 //   of 64 + 64 (-25 %).  Each pair still runs its own cta_group::2 MMA from its own leader; a smem stage is written by
 //   CTAs of BOTH pairs, so empty[s] counts one commit from each pair's leader (multicast to all four CTAs).
-template <int BN, class Epi, int CL = 1>
+// kOperand: kOperandBF16 (the name's case) or kOperandS8 (int8 x int8 -> s32; the similarity scans of int8 shards).
+template <int BN, class Epi, int CL = 1, int kOperand = kOperandBF16>
 __global__ void __launch_bounds__(128 + 32 * Epi::kEpiWarps, 1)
 gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, int M,
                     int N, int K, const __grid_constant__ typename Epi::Params ep, TileMap tmap) {
@@ -151,6 +172,8 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
   constexpr int kStages = Cfg::kStages;
   static_assert(CL == 1 || CL == 2 || CL == 4, "cluster size");
   constexpr bool kPair = CL >= 2;
+  constexpr bool kS8 = kOperand == kOperandS8;
+  constexpr int kBK = OperandTraits<kOperand>::kBK;
 
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -178,7 +201,7 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
   const int n_tiles = tmap.count((N + BN - 1) / BN);                // N-tiles this launch visits
   const int ksplit = tmap.ksplit;
   const int num_tiles = m_tiles * n_tiles * ksplit;  // work units
-  const int num_kb = (K + kGemmBK - 1) / kGemmBK;
+  const int num_kb = (K + kBK - 1) / kBK;
   const int kb_per = (num_kb + ksplit - 1) / ksplit;  // k-blocks per slice (the host keeps every slice non-empty)
 
   if (warp == kWarpProducer && lane == 0) {
@@ -235,21 +258,21 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
             // my A rows and my half of the B tile land in MY smem; the bytes are accounted on the pair leader's barrier
             const uint32_t leader_full = mapa_shared(smem_u32(&full_bar[stage]), crank & ~1u);
             if (prank == 0) mbar_expect_tx(&full_bar[stage], 2 * Cfg::kStageBytes);
-            tma_load_2d_pair(sa, &tma_a, leader_full, kb * kGemmBK, m0);
+            tma_load_2d_pair(sa, &tma_a, leader_full, kb * kBK, m0);
             if (CL == 2) {
-              tma_load_2d_pair(sb, &tma_b, leader_full, kb * kGemmBK, n0 + static_cast<int>(prank) * (BN / 2));
+              tma_load_2d_pair(sb, &tma_b, leader_full, kb * kBK, n0 + static_cast<int>(prank) * (BN / 2));
             } else {
               // quarter (crank >> 1) of my pair-rank's half of the weight tile, multicast to the CTA of my parity in both
               // pairs (same smem offset there); each destination accounts the bytes on ITS pair leader's full barrier
               const int quarter = static_cast<int>(crank >> 1);
               tma_load_2d_pair_multicast(sb + quarter * (BN / 4) * 128, &tma_b, leader_full,
-                                         kb * kGemmBK, n0 + static_cast<int>(prank) * (BN / 2) + quarter * (BN / 4),
+                                         kb * kBK, n0 + static_cast<int>(prank) * (BN / 2) + quarter * (BN / 4),
                                          static_cast<uint16_t>(0x5u << prank));
             }
           } else {
             mbar_expect_tx(&full_bar[stage], Cfg::kStageBytes);
-            tma_load_2d(sa, &tma_a, &full_bar[stage], kb * kGemmBK, m0);
-            tma_load_2d(sb, &tma_b, &full_bar[stage], kb * kGemmBK, n0);
+            tma_load_2d(sa, &tma_a, &full_bar[stage], kb * kBK, m0);
+            tma_load_2d(sb, &tma_b, &full_bar[stage], kb * kBK, n0);
           }
           if (++stage == kStages) { stage = 0; phase ^= 1; }
         }
@@ -258,7 +281,8 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
   } else if (warp == kWarpMma) {
     // ===================== MMA issuer =====================
     if (lane == 0 && prank == 0) {
-      constexpr uint32_t idesc = make_idesc_bf16(kGemmBM * (kPair ? 2 : 1), BN, false);
+      constexpr uint32_t idesc =
+          kS8 ? make_idesc_s8(kGemmBM * (kPair ? 2 : 1), BN) : make_idesc_bf16(kGemmBM * (kPair ? 2 : 1), BN, false);
       // commit masks: my pair's two CTAs; the smem stages of a 4-CTA cluster are shared by both pairs
       const uint16_t pair_mask = static_cast<uint16_t>(0x3u << (crank & ~1u));
       const uint16_t stage_mask = (CL == 4) ? static_cast<uint16_t>(0xF) : pair_mask;
@@ -281,9 +305,15 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_cons
           const uint64_t db = make_smem_desc_sw128(sb, 16, 1024);
 #pragma unroll
           for (int k = 0; k < kGemmBK / 16; ++k) {
-            // advance 16 bf16 = 32 B along K inside the 128-B swizzle row: +2 in the (addr >> 4) field
-            if (kPair) umma_bf16_ss_pair(tmem_d, da + 2 * k, db + 2 * k, idesc, ((kb - kb_begin) | k) != 0);
-            else umma_bf16_ss(tmem_d, da + 2 * k, db + 2 * k, idesc, ((kb - kb_begin) | k) != 0);
+            // advance 16 bf16 = 32 B along K inside the 128-B swizzle row: +2 in the (addr >> 4) field (int8: 32 values,
+            // the same 32 B)
+            if constexpr (kS8) {
+              if (kPair) umma_s8_ss_pair(tmem_d, da + 2 * k, db + 2 * k, idesc, ((kb - kb_begin) | k) != 0);
+              else umma_s8_ss(tmem_d, da + 2 * k, db + 2 * k, idesc, ((kb - kb_begin) | k) != 0);
+            } else {
+              if (kPair) umma_bf16_ss_pair(tmem_d, da + 2 * k, db + 2 * k, idesc, ((kb - kb_begin) | k) != 0);
+              else umma_bf16_ss(tmem_d, da + 2 * k, db + 2 * k, idesc, ((kb - kb_begin) | k) != 0);
+            }
           }
           // frees this smem stage (in both CTAs of a pair) once the MMAs above have read it
           if (kPair) umma_commit_pair(&empty_bar[stage], stage_mask);
@@ -969,13 +999,16 @@ __device__ __forceinline__ float2 slab_read(uint32_t slab, int r, int lane) {
 }
 
 // scores_f32[q, doc] = fixnan(acc * row_scale[q] * col_scale[doc])       (cos_sim / dot_score, NaN -> -1)
-struct OpScoresF32 {
-  struct Params {
-    float* out;
-    const float* row_scale;  // per query  (1/||q|| for cos_sim; null = 1)
-    const float* col_scale;  // per doc    (1/||d|| for cos_sim; null = 1)
-    long long ldc;
-  };
+// (kS8: the staged accumulator holds s32 values of an int8 launch, converted to fp32 before the scaling)
+struct ScoresF32Params {
+  float* out;
+  const float* row_scale;  // per query  (1/||q|| for cos_sim; null = 1)
+  const float* col_scale;  // per doc    (1/||d|| for cos_sim; null = 1)
+  long long ldc;
+};
+template <bool kS8 = false>
+struct OpScoresF32T {
+  using Params = ScoresF32Params;
   static __device__ __forceinline__ void rows(const Params& p, uint32_t slab, int m0, int rows, int col, int N,
                                               int lane) {
     const bool ok0 = col < N, ok1 = col + 1 < N;
@@ -996,7 +1029,7 @@ struct OpScoresF32 {
 #pragma unroll
       for (int u = 0; u < 8; ++u) {
         const float rs = __shfl_sync(0xffffffffu, my_rs, r + u);
-        float x = a[u].x * rs * c0, y = a[u].y * rs * c1;
+        float x = acc_to_f32<kS8>(__float_as_uint(a[u].x)) * rs * c0, y = acc_to_f32<kS8>(__float_as_uint(a[u].y)) * rs * c1;
         x = (x != x) ? -1.f : x;
         y = (y != y) ? -1.f : y;
         if (vec) *reinterpret_cast<float2*>(dst) = make_float2(x, y);
@@ -1010,7 +1043,7 @@ struct OpScoresF32 {
     for (; r < rows; ++r) {
       const float rs = __shfl_sync(0xffffffffu, my_rs, r);
       const float2 a = slab_read(slab, r, lane);
-      float x = a.x * rs * c0, y = a.y * rs * c1;
+      float x = acc_to_f32<kS8>(__float_as_uint(a.x)) * rs * c0, y = acc_to_f32<kS8>(__float_as_uint(a.y)) * rs * c1;
       x = (x != x) ? -1.f : x;
       y = (y != y) ? -1.f : y;
       if (vec) *reinterpret_cast<float2*>(dst) = make_float2(x, y);
@@ -1022,6 +1055,7 @@ struct OpScoresF32 {
     }
   }
 };
+using OpScoresF32 = OpScoresF32T<false>;
 
 // Threshold filter of the fused search (search.cu): score = fixnan(acc * row_scale[q] * col_scale[doc]); every score
 // >= tau[q] is appended as a packed (score bits, local doc index) pair to a candidate list; the score matrix itself is
@@ -1041,25 +1075,27 @@ struct OpScoresF32 {
 // score of a distinct real document, so the k-th largest of a query's maxima is a valid lower bound of its final k-th
 // best score — at a quarter of the entries (and no document indices) the full sample would need.  Slots this thread never
 // fills are written as 0xffffffff (maps to the invalid key 0 of the selection kernels).
-struct EpiFilterRows {
-  struct Params {
-    const float* row_scale;  // [M] or null
-    const float* col_scale;  // [N] or null
-    const float* tau;        // [M] per-query admission threshold; null -> admit everything
-    const float* tau_hi;     // [M] upper threshold (>= tau) or null: scores >= tau_hi are appended at the FRONT of the list,
-                             // scores in [tau, tau_hi) at its BACK (filled downwards from slot L - 1); null -> all front
-    uint2* cand;             // [M][groups][L]
-    int* counts;             // [groups][M] front entries
-    int* counts_back;        // [groups][M] back entries (only with tau_hi)
-    long long stride_q;      // entries between consecutive queries' list blocks
-    int L;                   // entries per (query, group) list
-    int group0;              // first group index this launch writes
-    int nq;
-    float* pool;             // sample mode: [M][groups][Lp] block maxima (cand / counts / tau unused)
-    long long stride_p;      // floats between consecutive queries' blocks of `pool`
-    int Lp;                  // floats per (query, group): 32 x tiles per CTA
-    int pair;                // 1: launched as CTA pairs (cta_group::2, M = 256 queries per scan)
-  };
+struct FilterRowsParams {
+  const float* row_scale;  // [M] or null
+  const float* col_scale;  // [N] or null
+  const float* tau;        // [M] per-query admission threshold; null -> admit everything
+  const float* tau_hi;     // [M] upper threshold (>= tau) or null: scores >= tau_hi are appended at the FRONT of the list,
+                           // scores in [tau, tau_hi) at its BACK (filled downwards from slot L - 1); null -> all front
+  uint2* cand;             // [M][groups][L]
+  int* counts;             // [groups][M] front entries
+  int* counts_back;        // [groups][M] back entries (only with tau_hi)
+  long long stride_q;      // entries between consecutive queries' list blocks
+  int L;                   // entries per (query, group) list
+  int group0;              // first group index this launch writes
+  int nq;
+  float* pool;             // sample mode: [M][groups][Lp] block maxima (cand / counts / tau unused)
+  long long stride_p;      // floats between consecutive queries' blocks of `pool`
+  int Lp;                  // floats per (query, group): 32 x tiles per CTA
+  int pair;                // 1: launched as CTA pairs (cta_group::2, M = 256 queries per scan)
+};
+template <bool kS8>  // kS8: s32 accumulator of an int8 launch
+struct EpiFilterRowsT {
+  using Params = FilterRowsParams;
   struct State {
     int cnt;    // front entries (sample mode: maxima written)
     int cnt_b;  // back entries
@@ -1144,12 +1180,12 @@ struct EpiFilterRows {
       if (nan_path) {
 #pragma unroll
         for (int i = 0; i < 32; ++i) {
-          const float s = __uint_as_float(v[i]) * rs * cs[i];
+          const float s = acc_to_f32<kS8>(v[i]) * rs * cs[i];
           x[i] = (s != s) ? -1.f : s;
         }
       } else {
 #pragma unroll
-        for (int i = 0; i < 32; ++i) x[i] = __uint_as_float(v[i]) * rs * cs[i];
+        for (int i = 0; i < 32; ++i) x[i] = acc_to_f32<kS8>(v[i]) * rs * cs[i];
       }
       if (pooled) {
         // sample pass: maxima of 4 consecutive documents, two 16-byte stores (cnt is a multiple of 8, the lists 32-byte
@@ -1194,6 +1230,8 @@ struct EpiFilterRows {
     st.cnt_b = cnt_b;
   }
 };
+using EpiFilterRows = EpiFilterRowsT<false>;
+using EpiFilterRowsS8 = EpiFilterRowsT<true>;
 using EpiFilterCandidates = EpiFilterRows;
 
 
@@ -1238,5 +1276,6 @@ struct EpiDebugNull {
   }
 };
 using EpiScoresF32 = EpiStaged<OpScoresF32>;
+using EpiScoresF32S8 = EpiStaged<OpScoresF32T<true>>;
 
 }  // namespace sgpt

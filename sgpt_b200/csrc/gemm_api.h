@@ -19,16 +19,22 @@ FilterGeometry filter_geometry(long long tiles, int nq);
 // index) to the list cand[q * stride_q + (group0 + g) * L + ...] — scores >= tau_hi[q] at its front, the others at its
 // back (tau_hi == nullptr: all at the front) — and writes counts / counts_back[(group0 + g) * nq + q] for the groups g of
 // this launch (filter_geometry of the visited tile count).  tile_mode/tile_stride select the corpus tiles visited
-// (gemm.cuh TileMap).  nq <= 256 (above 128: CTA pairs, M = 256).
+// (gemm.cuh TileMap).  nq <= 256 (above 128: CTA pairs, M = 256).  elem: SGPT_ELEM_BF16 or SGPT_ELEM_I8 (Q and C both
+// of that type; int8 launches take the s32 accumulator through the same scaling).
 int launch_filter_candidates(const void* Q, const void* C, const float* q_scale, const float* c_scale,
                              const float* tau, const float* tau_hi, uint2* cand, int* counts, int* counts_back,
-                             long long stride_q, int L, int group0, int nq, int n, int D, int tile_mode, int tile_stride,
-                             cudaStream_t stream);
+                             long long stride_q, int L, int group0, int nq, int n, int D, int elem, int tile_mode,
+                             int tile_stride, cudaStream_t stream);
 
 // The same GEMM over every tile_stride-th corpus tile in sample mode: pool[q * stride_p + g * Lp + ...] receives the
 // maximum score of every 4 consecutive documents the group visited (filter_geometry(sampled tiles).L / 4 floats per list,
 // unused slots = 0xffffffff).  Input of launch_tau_select (topk.cuh).
 int launch_sample_maxima(const void* Q, const void* C, const float* q_scale, const float* c_scale, float* pool,
-                         long long stride_p, int Lp, int nq, int n, int D, int tile_stride, cudaStream_t stream);
+                         long long stride_p, int Lp, int nq, int n, int D, int elem, int tile_stride,
+                         cudaStream_t stream);
+
+// sgpt_scores for either element type: scores[q, j] = fixnan(acc * q_scale[q] * c_scale[j]) as fp32 [nq, lds].
+int launch_scores(const void* Q, const void* C, const float* q_scale, const float* c_scale, float* scores, int64_t lds,
+                  int nq, int64_t n, int D, int elem, cudaStream_t stream);
 
 }  // namespace sgpt

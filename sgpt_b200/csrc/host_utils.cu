@@ -44,6 +44,10 @@ int make_tma_2d_f32(CUtensorMap* map, const void* base, uint64_t rows, uint64_t 
                     uint32_t box_cols) {
   return make_tma_2d(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, base, rows, cols, ld, box_rows, box_cols);
 }
+int make_tma_2d_u8(CUtensorMap* map, const void* base, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows,
+                   uint32_t box_cols) {
+  return make_tma_2d(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, base, rows, cols, ld, box_rows, box_cols);
+}
 
 static int make_tma_2d(CUtensorMap* map, CUtensorMapDataType dt, uint64_t esz, const void* base, uint64_t rows,
                        uint64_t cols, uint64_t ld, uint32_t box_rows, uint32_t box_cols) {

@@ -35,6 +35,9 @@ int make_tma_2d_bf16(CUtensorMap* map, const void* base, uint64_t rows, uint64_t
 // Same for fp32 elements (box_cols = 32 floats = 128 B).
 int make_tma_2d_f32(CUtensorMap* map, const void* base, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows,
                     uint32_t box_cols);
+// 1-byte elements (int8 corpus shards and queries)
+int make_tma_2d_u8(CUtensorMap* map, const void* base, uint64_t rows, uint64_t cols, uint64_t ld, uint32_t box_rows,
+                   uint32_t box_cols);
 
 int sm_count();  // multiprocessors of the CURRENT device (cached per device)
 

@@ -99,9 +99,19 @@ extern "C" int64_t sgpt_search_workspace_bytes(int nq, int64_t n, int k) {
 
 // One shard, all query blocks.  `fin` carries the packed destinations of the final selection (TopkExtra::dst/flag:
 // this rank's buffer and/or peer gather buffers); out_scores / out_ids may be null when only those are wanted.
+// Checks of the element type shared by the _ex entry points; they run before any CUDA call.
+static int check_elem(const char* who, int elem, int D) {
+  SGPT_REQUIRE(elem == SGPT_ELEM_BF16 || elem == SGPT_ELEM_I8, "%s: unknown element type %d", who, elem);
+  // int8 rows: the TMA row pitch (D bytes) must be a multiple of 16, and |acc| <= 127^2 D must fit in int32
+  SGPT_REQUIRE(elem != SGPT_ELEM_I8 || (D > 0 && D % 16 == 0 && D <= 65536),
+               "%s: int8 rows need D a positive multiple of 16 and <= 65536 (D=%d)", who, D);
+  return SGPT_OK;
+}
+
+// (elem: SGPT_ELEM_BF16 / SGPT_ELEM_I8, checked by the callers; plan and workspace do not depend on it)
 static int search_impl(const void* Q, const void* Cm, const float* q_scale, const float* c_scale, int nq, int64_t n, int D,
                        int k, int64_t id_base, float* out_scores, int64_t* out_ids, void* ws, int64_t ws_bytes,
-                       const TopkExtra& fin, cudaStream_t stream) {
+                       const TopkExtra& fin, int elem, cudaStream_t stream) {
   SGPT_REQUIRE(nq >= 0 && n >= 0 && k > 0, "sgpt_search: bad sizes nq=%d n=%lld k=%d", nq, (long long)n, k);
   SGPT_REQUIRE(n < (1ll << 31), "sgpt_search: shard too large for one launch (n=%lld)", (long long)n);
   SGPT_REQUIRE(D > 0 && D % 8 == 0, "sgpt_search: D=%d must be a positive multiple of 8", D);
@@ -117,10 +127,11 @@ static int search_impl(const void* Q, const void* Cm, const float* q_scale, cons
         f.dst[p] += static_cast<size_t>(q0) * k;
         if (f.flag[p] != nullptr) f.flag[p] += q0;
       }
-      int rc = search_impl(static_cast<const uint8_t*>(Q) + static_cast<size_t>(q0) * D * 2, Cm,
+      const size_t row_bytes = static_cast<size_t>(D) * (elem == SGPT_ELEM_I8 ? 1 : 2);
+      int rc = search_impl(static_cast<const uint8_t*>(Q) + static_cast<size_t>(q0) * row_bytes, Cm,
                            q_scale ? q_scale + q0 : nullptr, c_scale, nb, n, D, k, id_base,
                            out_scores ? out_scores + static_cast<size_t>(q0) * k : nullptr,
-                           out_ids ? out_ids + static_cast<size_t>(q0) * k : nullptr, ws, ws_bytes, f, stream);
+                           out_ids ? out_ids + static_cast<size_t>(q0) * k : nullptr, ws, ws_bytes, f, elem, stream);
       if (rc != SGPT_OK) return rc;
     }
     return SGPT_OK;
@@ -129,7 +140,7 @@ static int search_impl(const void* Q, const void* Cm, const float* q_scale, cons
   if (!p.two_pass) {
     float* scores = static_cast<float*>(ws);
     const int64_t lds = padded_cols(n);
-    int rc = sgpt_scores(Q, Cm, q_scale, c_scale, scores, lds, nq, n, D, stream);
+    int rc = launch_scores(Q, Cm, q_scale, c_scale, scores, lds, nq, n, D, elem, stream);
     if (rc != SGPT_OK) return rc;
     TopkSrc src{};
     src.scores = scores;
@@ -157,13 +168,14 @@ static int search_impl(const void* Q, const void* Cm, const float* q_scale, cons
   int* need_generic = reinterpret_cast<int*>(w);
 
   // pass A: block maxima of the sampled tiles -> admission thresholds
-  int rc = launch_sample_maxima(Q, Cm, q_scale, c_scale, pool, p.stride_p, p.Lp, nq, static_cast<int>(n), D, p.stride, stream);
+  int rc = launch_sample_maxima(Q, Cm, q_scale, c_scale, pool, p.stride_p, p.Lp, nq, static_cast<int>(n), D, elem,
+                                p.stride, stream);
   if (rc != SGPT_OK) return rc;
   rc = launch_tau_select(pool, p.stride_p, static_cast<int>(p.stride_p), nq, k, p.k_hi, tau, tau_hi, stream);
   if (rc != SGPT_OK) return rc;
   // pass B: the whole shard, admission threshold tau[q], front / back split at tau_hi[q]
   rc = launch_filter_candidates(Q, Cm, q_scale, c_scale, tau, tau_hi, cand, cnt, cnt_back, p.stride_b, p.gb.L, 0, nq,
-                                static_cast<int>(n), D, /*tile_mode=*/0, 1, stream);
+                                static_cast<int>(n), D, elem, /*tile_mode=*/0, 1, stream);
   if (rc != SGPT_OK) return rc;
   // final exact selection over the candidates
   TopkSrc src{};
@@ -184,17 +196,26 @@ static int search_impl(const void* Q, const void* Cm, const float* q_scale, cons
   return launch_topk_select(src, nq, k, out_scores, out_ids, stream, fin);
 }
 
-extern "C" int sgpt_search(const void* Q, const void* Cm, const float* q_scale, const float* c_scale, int nq,
-                           int64_t n, int D, int k, int64_t id_base, float* out_scores, int64_t* out_ids, void* ws,
-                           int64_t ws_bytes, sgpt_stream_t stream_) {
+extern "C" int sgpt_search_ex(const void* Q, const void* Cm, const float* q_scale, const float* c_scale, int nq,
+                              int64_t n, int D, int k, int64_t id_base, float* out_scores, int64_t* out_ids, void* ws,
+                              int64_t ws_bytes, int elem, sgpt_stream_t stream_) {
+  if (int rc = check_elem("sgpt_search", elem, D)) return rc;
   SGPT_REQUIRE(nq == 0 || (out_scores != nullptr && out_ids != nullptr), "sgpt_search: null output");
-  return search_impl(Q, Cm, q_scale, c_scale, nq, n, D, k, id_base, out_scores, out_ids, ws, ws_bytes, TopkExtra(),
+  return search_impl(Q, Cm, q_scale, c_scale, nq, n, D, k, id_base, out_scores, out_ids, ws, ws_bytes, TopkExtra(), elem,
                      static_cast<cudaStream_t>(stream_));
 }
 
-extern "C" int sgpt_search_packed(const void* Q, const void* Cm, const float* q_scale, const float* c_scale, int nq,
-                                  int64_t n, int D, int k, int64_t id_base, uint64_t* out_packed, void* ws,
-                                  int64_t ws_bytes, sgpt_stream_t stream_) {
+extern "C" int sgpt_search(const void* Q, const void* Cm, const float* q_scale, const float* c_scale, int nq,
+                           int64_t n, int D, int k, int64_t id_base, float* out_scores, int64_t* out_ids, void* ws,
+                           int64_t ws_bytes, sgpt_stream_t stream_) {
+  return sgpt_search_ex(Q, Cm, q_scale, c_scale, nq, n, D, k, id_base, out_scores, out_ids, ws, ws_bytes, SGPT_ELEM_BF16,
+                        stream_);
+}
+
+extern "C" int sgpt_search_packed_ex(const void* Q, const void* Cm, const float* q_scale, const float* c_scale, int nq,
+                                     int64_t n, int D, int k, int64_t id_base, uint64_t* out_packed, void* ws,
+                                     int64_t ws_bytes, int elem, sgpt_stream_t stream_) {
+  if (int rc = check_elem("sgpt_search_packed", elem, D)) return rc;
   SGPT_REQUIRE(nq == 0 || out_packed != nullptr, "sgpt_search_packed: null output");
   SGPT_REQUIRE(id_base >= 0 && id_base + n < (1ll << 31), "sgpt_search_packed: global ids must fit 31 bits (id_base=%lld n=%lld)",
                (long long)id_base, (long long)n);
@@ -203,8 +224,15 @@ extern "C" int sgpt_search_packed(const void* Q, const void* Cm, const float* q_
   fin.n_dst = 1;
   fin.dst_slot = 0;
   fin.dst_nq = nq;
-  return search_impl(Q, Cm, q_scale, c_scale, nq, n, D, k, id_base, nullptr, nullptr, ws, ws_bytes, fin,
+  return search_impl(Q, Cm, q_scale, c_scale, nq, n, D, k, id_base, nullptr, nullptr, ws, ws_bytes, fin, elem,
                      static_cast<cudaStream_t>(stream_));
+}
+
+extern "C" int sgpt_search_packed(const void* Q, const void* Cm, const float* q_scale, const float* c_scale, int nq,
+                                  int64_t n, int D, int k, int64_t id_base, uint64_t* out_packed, void* ws,
+                                  int64_t ws_bytes, sgpt_stream_t stream_) {
+  return sgpt_search_packed_ex(Q, Cm, q_scale, c_scale, nq, n, D, k, id_base, out_packed, ws, ws_bytes, SGPT_ELEM_BF16,
+                               stream_);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -282,11 +310,12 @@ extern "C" void sgpt_gather_destroy(sgpt_gather_t g) {
   delete g;
 }
 
-extern "C" int sgpt_search_gather(sgpt_gather_t g, const void* Q, const void* Cm, const float* q_scale,
-                                  const float* c_scale, int nq, int64_t n, int D, int k, int64_t id_base,
-                                  const int64_t* exclude_ids, float* out_scores, int64_t* out_ids, void* ws,
-                                  int64_t ws_bytes, sgpt_stream_t stream_) {
+extern "C" int sgpt_search_gather_ex(sgpt_gather_t g, const void* Q, const void* Cm, const float* q_scale,
+                                     const float* c_scale, int nq, int64_t n, int D, int k, int64_t id_base,
+                                     const int64_t* exclude_ids, float* out_scores, int64_t* out_ids, void* ws,
+                                     int64_t ws_bytes, int elem, sgpt_stream_t stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  if (int rc = check_elem("sgpt_search_gather", elem, D)) return rc;
   SGPT_REQUIRE(g != nullptr, "sgpt_search_gather: null gather context");
   SGPT_REQUIRE(nq >= 0 && nq <= g->nq_cap && k == g->k, "sgpt_search_gather: nq=%d k=%d do not fit the context (nq<=%d, k=%d)",
                nq, k, g->nq_cap, g->k);
@@ -306,7 +335,7 @@ extern "C" int sgpt_search_gather(sgpt_gather_t g, const void* Q, const void* Cm
     fin.dst[r] = reinterpret_cast<uint2*>(g->peers[r] + static_cast<size_t>(par) * g->parity_bytes);
     fin.flag[r] = reinterpret_cast<unsigned int*>(g->peers[r] + flag_off);
   }
-  int rc = search_impl(Q, Cm, q_scale, c_scale, nq, n, D, k, id_base, nullptr, nullptr, ws, ws_bytes, fin, stream);
+  int rc = search_impl(Q, Cm, q_scale, c_scale, nq, n, D, k, id_base, nullptr, nullptr, ws, ws_bytes, fin, elem, stream);
   // the counters of this parity are consumed whether or not the merge below is launched
   g->uses[par] += 1;
   g->calls += 1;
@@ -324,6 +353,14 @@ extern "C" int sgpt_search_gather(sgpt_gather_t g, const void* Q, const void* Cm
   src.wait_flag = reinterpret_cast<const unsigned int*>(g->local + flag_off);
   src.wait_target = target;
   return launch_topk_select(src, nq, k, out_scores, out_ids, stream);
+}
+
+extern "C" int sgpt_search_gather(sgpt_gather_t g, const void* Q, const void* Cm, const float* q_scale,
+                                  const float* c_scale, int nq, int64_t n, int D, int k, int64_t id_base,
+                                  const int64_t* exclude_ids, float* out_scores, int64_t* out_ids, void* ws,
+                                  int64_t ws_bytes, sgpt_stream_t stream_) {
+  return sgpt_search_gather_ex(g, Q, Cm, q_scale, c_scale, nq, n, D, k, id_base, exclude_ids, out_scores, out_ids, ws,
+                               ws_bytes, SGPT_ELEM_BF16, stream_);
 }
 
 extern "C" int sgpt_topk_merge_packed(const uint64_t* in_packed, int G, int nq, int k, float* out_scores,

@@ -87,11 +87,12 @@ class PeerGather:
         out_s = torch.empty((nq, k), dtype=torch.float32, device=self.device)
         out_i = torch.empty((nq, k), dtype=torch.int64, device=self.device)
         with torch.cuda.device(self.device):
-            rc = self._lib.sgpt_search_gather(self._handle, qb.data_ptr(), shard.vectors.data_ptr(), _lib.ptr(q_scale),
-                                              c_scale, nq, shard.n, shard.dim, k, shard.id_base, _lib.ptr(exclude_ids),
-                                              out_s.data_ptr(), out_i.data_ptr(), shard._ws.data_ptr(),
-                                              shard._ws.numel(), _lib.current_stream())
-        _lib.check(rc, "sgpt_search_gather")
+            rc = self._lib.sgpt_search_gather_ex(self._handle, qb.data_ptr(), shard.vectors.data_ptr(),
+                                                 _lib.ptr(q_scale), c_scale, nq, shard.n, shard.dim, k, shard.id_base,
+                                                 _lib.ptr(exclude_ids), out_s.data_ptr(), out_i.data_ptr(),
+                                                 shard._ws.data_ptr(), shard._ws.numel(), shard._elem,
+                                                 _lib.current_stream())
+        _lib.check(rc, "sgpt_search_gather_ex")
         return out_s, out_i
 
     def close(self):
@@ -141,8 +142,9 @@ class ShardedDenseRetrievalExactSearch:
 
     def __init__(self, model, batch_size: int = 128, corpus_chunk_size: int = 50000, group=None,
                  shard_factory: Optional[Callable] = None, merge: Optional[Callable] = None, peer_gather: bool = False,
-                 **kwargs):
+                 corpus_dtype: str = "bf16", **kwargs):
         self.model, self.batch_size, self.corpus_chunk_size = model, batch_size, corpus_chunk_size
+        self.corpus_dtype = corpus_dtype  # element type of the resident shards: "bf16" or "int8" (CorpusShard dtype)
         self.group, self.shard_factory, self.merge = group, shard_factory, merge
         self.peer_gather = peer_gather  # exchange through NVLink peer mappings (PeerGather) instead of one NCCL all-gather
         self.show_progress_bar, self.convert_to_tensor = True, True
@@ -174,7 +176,8 @@ class ShardedDenseRetrievalExactSearch:
             from .index import CorpusShard
 
             # the shard numbers its rows rank * cap + j, so a merged id still names its owner: (id // cap, id % cap)
-            shard = CorpusShard(q_emb.shape[1], max(len(mine), 1), device=self.device, id_base=rank * cap)
+            shard = CorpusShard(q_emb.shape[1], max(len(mine), 1), device=self.device, id_base=rank * cap,
+                                dtype=self.corpus_dtype)
         else:
             shard = self.shard_factory(q_emb.shape[1], max(len(mine), 1))
         for batch_num, start in enumerate(range(0, len(mine), self.corpus_chunk_size)):

@@ -20,13 +20,15 @@ logger = logging.getLogger(__name__)
 
 class DenseRetrievalExactSearch:
     def __init__(self, model, batch_size: int = 128, corpus_chunk_size: int = 50000, plain_lists: bool = False,
-                 **kwargs):
+                 corpus_dtype: str = "bf16", **kwargs):
         """model is any class that provides encode_corpus() and encode_queries() (XS:24).  ``plain_lists=False`` is the
         reference's custom convention — ``[(id, text)]`` / ``[(id, {title, text})]`` tuples and a ``batch_num`` keyword
         (XS:56-62, 87-93); ``plain_lists=True`` is upstream beir's DRES convention — ``List[str]`` /
         ``List[{title, text}]`` — which the ST-path wrappers (SentenceBERTBOSEOS / SentenceBERTAsym, used with
-        ``beir.retrieval.search.dense.DenseRetrievalExactSearch`` at BDR:405-412) expect."""
+        ``beir.retrieval.search.dense.DenseRetrievalExactSearch`` at BDR:405-412) expect.  ``corpus_dtype`` is the
+        element type the corpus chunks are searched in: "bf16" or "int8" (per-row int8 rows, see CorpusShard)."""
         self.model = model
+        self.corpus_dtype = corpus_dtype
         self.plain_lists = plain_lists
         self.batch_size = batch_size
         self.score_functions = {"cos_sim": "cos_sim", "dot": "dot"}
@@ -75,7 +77,7 @@ class DenseRetrievalExactSearch:
             sub = self._as_device(self.model.encode_corpus(
                 corpus_list[start:end], batch_size=self.batch_size, show_progress_bar=self.show_progress_bar,
                 convert_to_tensor=self.convert_to_tensor, **extra))
-            shard = CorpusShard.from_embeddings(sub, device=self.device, id_base=start)
+            shard = CorpusShard.from_embeddings(sub, device=self.device, id_base=start, dtype=self.corpus_dtype)
             # XS:96-108: scores, NaN -> -1, top-(k+1) of this chunk
             s, i = shard.search(q_emb, kk, score_function)
             # XS:112-132: drop self matches, merge with the running lists, keep the best k+1

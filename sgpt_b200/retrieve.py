@@ -40,6 +40,8 @@ def parse_args(argv=None):
     p.add_argument("--specb", action="store_const", default=False, const=True, help="Use special brackets encoding method")
     p.add_argument("--maxseqlen", type=int, default=None, help="Sequence length to use; SGPT-msmarco-specb models use 300")
     p.add_argument("--outdir", type=str, default=".", help="Where the result JSON files are written (reference: cwd)")
+    p.add_argument("--corpusdtype", type=str, default="bf16", choices=["bf16", "int8"],
+                   help="Element type of the searched corpus embeddings: bf16, or int8 rows with one scale per row")
     return p.parse_args(argv)
 
 
@@ -65,12 +67,14 @@ def build_retriever(args):
         else:
             wrapped = _PlainSentenceBERT(model)
         wrapped.device = model.device
-        return DenseRetrievalExactSearch(wrapped, batch_size=args.batchsize, plain_lists=True)
+        return DenseRetrievalExactSearch(wrapped, batch_size=args.batchsize, plain_lists=True,
+                                         corpus_dtype=args.corpusdtype)
     if args.speca:
         raise ValueError("speca is only supported with use_st")  # BDR:415-416
     return DenseRetrievalExactSearch(CustomEmbedder(
         model_name=args.modelname, method=args.method, device=args.device, batch_size=args.batchsize,
-        save_emb=args.saveemb, layeridx=args.layeridx, specb=args.specb, maxseqlen=args.maxseqlen, dataset=args.dataset))
+        save_emb=args.saveemb, layeridx=args.layeridx, specb=args.specb, maxseqlen=args.maxseqlen, dataset=args.dataset),
+        corpus_dtype=args.corpusdtype)
 
 
 class _PlainSentenceBERT:
